@@ -27,6 +27,7 @@ from wb_humanoid_mpc_b200 import abi, model_loader, references  # noqa: E402
 
 METRIC = "SQP solves/sec (G1 whole-body, N=100, batched)"
 SEED = 1234
+DUMP_BYTES = 60 << 20   # --dump-outputs stays under 64 MB, .npy headers included
 
 
 def build_batch(model, batch, rank, horizon, gaits, random_phase=False):
@@ -52,6 +53,24 @@ def build_batch(model, batch, rank, horizon, gaits, random_phase=False):
         insts.append(references.build_instance(model, x0, t0=0.0, horizon=horizon, gait=g, gait_start=start, cmd=cmd))
         insts[-1]["cmd"], insts[-1]["gait"] = cmd, g
     return insts
+
+
+def dump_outputs(out_dir, groups):
+    """--dump-outputs: writes what the timed path handed its caller in the last timed step as <out_dir>/<name><suffix>.npy in float64, so that
+    two builds can be compared output for output (the inputs are seeded).  groups = {suffix: {name: array with the instances along axis 0}}
+    (one group per node count in the mixed sweep).  Above DUMP_BYTES in all, the same seeded sample of every group's instances is written;
+    instance<suffix>.npy holds the indices of the instances written."""
+    rng = np.random.default_rng(SEED)
+    total = sum(8 * np.asarray(a).size for arrays in groups.values() for a in arrays.values())
+    frac = min(1.0, DUMP_BYTES / total)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for suffix, arrays in groups.items():
+        n = len(next(iter(arrays.values())))
+        keep = np.arange(n) if frac == 1.0 else np.sort(rng.choice(n, max(1, int(frac * n)), replace=False))
+        np.save(out / f"instance{suffix}.npy", keep.astype(np.float64))
+        for name, a in arrays.items():
+            np.save(out / f"{name}{suffix}.npy", np.asarray(a, dtype=np.float64)[keep])
 
 
 class ClockSampler:
@@ -280,6 +299,8 @@ def run_mixed(args, model, settings, rank, world, local_rank, workload, cores):
         sampler.start()
     dev_s = timed(resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"_n{g['n']}": g["solver"].primal_solution() for g in groups})
     launches = sum(g["solver"].launch_count() for g in groups) * args.steps
     stage = {str(g["n"]): dict(zip(["lq", "qp", "linesearch", "lq_projection_share"], [float(v) for v in g["solver"].benchmarks()])) for g in groups}
     each(e2e_step)
@@ -321,7 +342,11 @@ def main():
     ap.add_argument("--check-oracle", action="store_true", help="additionally cross-check the GPU solution against the (slow) checker oracle")
     ap.add_argument("--sqp-iteration", type=int, default=1, help="sqpIteration (1 = the shipped real-time iteration; 10 = the secondary number)")
     ap.add_argument("--global-step", action="store_true", help="one line-search step per iteration for the whole multi-GPU batch (NCCL)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the solutions of the last one (rank 0's instances) as "
+                                                          "DIR/<name>.npy, float64, at most 64 MB (a seeded sample of the instances above that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.batch <= 0:
         args.batch = 256 if args.config == "c3" else 1024
 
@@ -361,12 +386,15 @@ def main():
         cores = calibrate_threads(model, max(groups, key=len), settings, cores)
         times, stage = [], np.zeros(3)
         for _ in range(args.steps):
-            tstep = 0.0
+            tstep, last = 0.0, {}
             for g in groups:
                 o = cpu_port_solve(model, g, settings, cores)
                 tstep += o["seconds"]
                 stage += o["stage_s"]
+                last[f"_n{len(g[0]['t_nodes'])}" if args.config == "c5" else ""] = {k: o[k] for k in ("x", "u", "n_iter", "log")}
             times.append(tstep)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
         total = sum(times)
         val = sample * args.steps / total
         ta = [cpu_port_solve(model, insts[:1], settings, 1, node_threads=4)["seconds"] for _ in range(8)][3:]
@@ -453,6 +481,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     sol = solver.primal_solution()
     assert not sol["status"].any()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"": sol})
     alphas = sol["log"][:, 0, 8]
 
     # ---- end-to-end through the C ABI with host buffers (e2e) --------------------------------------------------------------------

@@ -263,17 +263,15 @@ def test_cpp_config_loader_equals_the_flat_model_file():
     """host/model_from_config.hpp reads the reference's OWN files (URDF + task.info + reference.info + gait.info: boost INFO subset, URDF subset,
     welded fixed joints, Pinocchio joint order, frames, weights) -- what a node passes to WBMpcInterface -- and must produce the HostModel the flat
     model file gives (that file is derived from the same config files by the Python loader, model_loader.py): every field of b200sqp_model_desc,
-    the settings, the reference-manager parameters and the gait table.  Needs the reference tree (absent on the GPU box: skipped there)."""
+    the settings, the reference-manager parameters and the gait table.  The config files are copies under tests/golden/g1_config."""
     import ctypes as C
     from pathlib import Path
 
     from wb_humanoid_mpc_b200 import host_lib, model_loader
 
-    root = Path("/root/reference")
+    root = Path(__file__).resolve().parent / "golden" / "g1_config"
     rel = model_loader.G1_REL
     files = [root / rel["urdf"], root / rel["task"], root / rel["reference"], root / rel["gait"]]
-    if not all(f.exists() for f in files):
-        pytest.skip("reference config files not present")
     a = host_lib.HostModel()                 # flat file
     b = host_lib.HostModel(config=files)     # C++ loader of the config files
     assert (a.nx, a.nu, a.dt, a.horizon) == (b.nx, b.nu, b.dt, b.horizon)
